@@ -29,15 +29,18 @@ offline: see DESIGN.md) and prints the same line with "impl": "reference".
 import argparse
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "decode_tokens_per_s"
 UNIT = "tokens/s"
@@ -278,12 +281,21 @@ def gpu_comparators(torch, ops, cfg, runner, weights, dev, ctx):
     BF16 = torch.bfloat16
     sc = D ** -0.5
     # ---- attention: FlashInfer fa2 -------------------------------------------------------------------------------
+    fi_tmp = tempfile.mkdtemp(prefix="xb_bench_flashinfer_")
     try:
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         import build_flashinfer_cache as FIC
-        FIC.set_env()
+        # FlashInfer writes a log, lock files (cached_ops/tmp) and JIT output under its workspace: give it a temporary one, with
+        # the modules pre-built in the tree linked in one by one
+        FIC.set_env(fi_tmp)
         import flashinfer
         from flashinfer.jit import core as jc
+        from flashinfer.jit import env as je
+        prebuilt = os.path.join(FIC.FI_BASE, os.path.relpath(je.FLASHINFER_JIT_DIR, fi_tmp))
+        os.makedirs(je.FLASHINFER_JIT_DIR, exist_ok=True)
+        for name in os.listdir(prebuilt) if os.path.isdir(prebuilt) else []:
+            if name != "tmp":
+                os.symlink(os.path.join(prebuilt, name), os.path.join(je.FLASHINFER_JIT_DIR, name))
         if not all(s.jit_library_path.exists() for s in FIC.specs((D,))):
             raise RuntimeError("FlashInfer modules not pre-built (tools/build_flashinfer_cache.py)")
         orig = jc.JitSpec.build
@@ -323,6 +335,8 @@ def gpu_comparators(torch, ops, cfg, runner, weights, dev, ctx):
         add(f"ragged causal prefill attention 4x{Sp} {HQ}/{HKV}x{D} vs FlashInfer fa2", t_o, t_t)
     except Exception as e:
         out.append({"name": "FlashInfer fa2 attention", "error": str(e)[:200]})
+    finally:
+        shutil.rmtree(fi_tmp, ignore_errors=True)
     # ---- linears: cuBLASLt bf16 and torch._scaled_mm fp8 at the four projection shapes, M = 8192 ----------------------
     try:
         import torch.nn.functional as F
@@ -422,6 +436,16 @@ def scale_target_llama70b(torch, dist, dev, rank, world, exchange, steps=8, warm
     return out
 
 
+def dump_outputs(out_dir, runner):
+    """what a caller of the timed decode step receives from its last replay: the logits (float32 [batch, vocab], every
+    vocabulary column) and the greedy next token ids (float64, exact).  Rank 0 only: under TP its logits are the gathered
+    ones; with several replicas, replica 0's."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), runner.logits.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "next_tokens.npy"), runner.next_tokens.cpu().numpy().astype(np.float64))
+
+
 # ----------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -436,6 +460,8 @@ def main():
     ap.add_argument("--tp", type=int, default=0, help="tensor-parallel degree (default: min(N, 4) for Qwen2-7B's 28 heads)")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"])
     ap.add_argument("--no-scale-target", action="store_true", help="skip the Llama-3-70B FP8 batch-32 ctx-8192 measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step returned (logits, "
+                                                          "next token ids) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -539,6 +565,8 @@ def main():
     ms = e0.elapsed_time(e1)
     log(f"timed region done: {ms:.1f} ms")
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, runner)
     # a graph replay does not pass through the library's launch counter: count the kernels in one step eagerly
     n0 = _lib.launch_count()
     runner.launch_step()

@@ -21,8 +21,9 @@ Parity pinning (SURVEY.md 8c):
     files line by line; the reference's own kernel tests (torch expressions, no
     stored vectors) are restated on the oracle in tests/test_oracle_reference_kats_cpu.py,
     and the reference's kernels THEMSELVES are compiled from its sources into
-    oracle/_ref/ (oracle/build_ref.py) for the GPU-side comparison of
-    tools/ref_kernel_parity.py / tests/test_gpu_zzz_ref_kernels.py
+    oracle/_ref/ (oracle/build_ref.py); their outputs on the cases of
+    tests/ref_kernel_cases.py are stored in tests/golden/ref_kernels.pt.gz, which
+    tests/test_gpu_zzz_ref_kernels.py compares the CUDA kernels with
   * MoE router -> pinned by the known answers of tests/core/layers/mlu/moe_gate_test.cpp:143-268
     (tests/test_moe_cpu.py); whole-model composition -> transformers' Qwen2 / Llama
     (tests/test_oracle_vs_transformers_cpu.py)

@@ -5,9 +5,8 @@ the only missing header is <glog/logging.h>, for which oracle/ref_stubs/ forward
 FlashInfer and the FP8 GEMM = CUTLASS are un-vendored third-party code and stay "unbuildable": DESIGN.md section 2.)
 
 Outputs only into oracle/_ref/ (git-ignored, shipped to the GPU box): libxllm_ref_kernels.so + the test binding
-xllm_ref_kernels_py.so (oracle/ref_binding.cpp).  TEST INFRASTRUCTURE: used by tools/ref_kernel_parity.py /
-tests/test_gpu_zzz_ref_kernels.py to compare this library's kernels with the reference's on a GPU.  Needs /root/reference, i.e. runs
-in the build container only; the GPU box uses the prebuilt files.
+xllm_ref_kernels_py.so (oracle/ref_binding.cpp).  TEST INFRASTRUCTURE: tests/golden/make_ref_kernel_golden.py runs them on a GPU
+and stores their outputs for tests/test_gpu_zzz_ref_kernels.py.  Needs the reference's sources.
   python -m oracle.build_ref [-f]"""
 import os
 import subprocess

@@ -13,10 +13,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 FI_BASE = os.path.join(ROOT, "baseline", "_fi")
 
 
-def set_env():
-    os.environ["FLASHINFER_WORKSPACE_BASE"] = FI_BASE
+def set_env(base=FI_BASE):
+    os.environ["FLASHINFER_WORKSPACE_BASE"] = base
     os.environ["FLASHINFER_CUDA_ARCH_LIST"] = "10.0a"
-    os.makedirs(FI_BASE, exist_ok=True)
+    os.makedirs(base, exist_ok=True)
 
 
 def specs(head_dims=(128, 64)):
